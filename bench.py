@@ -14,6 +14,7 @@ length is pinned, SURVEY.md §8d).  A bench "step" is one full pass of the hot p
 Data parallel, no data-path collective ("weak" scaling); NCCL is used once, to broadcast the weights from rank 0.
 
   python bench.py --gpus 1 --steps 5 --warmup 3
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   # + what the last timed step returned, as DIR/*.npy
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      # the reference's own CPU path (baseline/_ref when present, else the oracle port)
 """
@@ -83,6 +84,25 @@ def bench_texts(rank, B):
 
 def bench_ref_tokens():
     return torch.randint(0, 2048, (REF_FRAMES, 32), generator=torch.Generator().manual_seed(7))
+
+
+def dump_outputs(out_dir, toks, n_tok, wav_host, wav_len):
+    """Writes what the last timed step of each leg handed to its caller as DIR/<name>.npy, so that two builds can be
+    compared output for output: the resident leg's AR tokens and frame counts (exact in float32), and the API leg's
+    waveforms at one fixed, seeded set of sample positions shared by every utterance (zero past an utterance's end).
+    The sample keeps the waveforms to 32 MiB; the full ones are about 3 MB per utterance."""
+    os.makedirs(out_dir, exist_ok=True)
+    B, cols = wav_host.shape
+    k = min(cols, max(1, (32 << 20) // (4 * B)))
+    idx = np.sort(np.random.default_rng(0).choice(cols, k, replace=False))
+    lens = np.asarray(wav_len, dtype=np.int64)
+    wav = wav_host.numpy()[:, idx]
+    wav[idx[None, :] >= lens[:, None]] = 0.0
+    arrays = {"ar_tokens": toks.astype(np.float32), "ar_frames": n_tok.astype(np.float32),
+              "wav_samples": wav.astype(np.float32), "wav_sample_index": idx.astype(np.float64),
+              "wav_lengths": lens.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -396,7 +416,13 @@ def main():
     ap.add_argument("--batch", type=int, default=BATCH_PER_GPU, help="utterances per GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip batch-1 / TTFA / RTF / Mimi side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (rank 0, B200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the B200 arm's outputs; it does not apply to --impl reference")
     torch.set_grad_enabled(False)
     # Libraries (NCCL's version banner, ...) write to fd 1; the contract is ONE JSON line on stdout.
     # Everything else goes to stderr, the JSON is written to the real stdout at the end.
@@ -485,6 +511,7 @@ def main():
     all_texts = [t for r in range(max(world, 1)) for t in bench_texts(r, B)]
     all_seeds = list(range(1234, 1234 + len(all_texts)))
     wav_host = torch.empty((B, STEPS_AR * 1920), dtype=torch.float32).pin_memory()
+    wav_len = [0] * B  # samples of each utterance in wav_host after the last API pass
 
     def one_pass_resident():
         ses.begin(cond_d, txt_d, lens, noise_d, samp)
@@ -496,6 +523,7 @@ def main():
         for j, w in enumerate(wavs):  # the result in host memory
             n = int(w.shape[-1])
             wav_host[j, :n].copy_(w.reshape(-1), non_blocking=True)
+            wav_len[j] = n
             frames += n // 1920
         torch.cuda.current_stream(dev).synchronize()
         return frames
@@ -542,6 +570,8 @@ def main():
         e2e_ms += a.elapsed_time(b)
     clocks.stop_flag = True
     clocks.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, toks, n_tok, wav_host, wav_len)
     t = torch.tensor([t_total_ms, e2e_ms, t_kernel_ms], dtype=torch.float64, device=dev)
     fr = torch.tensor([float(frames_per_pass), float(e2e_frames)], dtype=torch.float64, device=dev)
     if world > 1:
