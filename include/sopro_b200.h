@@ -424,7 +424,7 @@ int sopro_nar_set_graphs(sopro_nar_t* n, int enabled);
 
 /* ------------------------------------------------------------------------------------------------
  * Prefill: SoproTTSModel.prepare_conditioning (reference model.py:172-216) for B texts that share one prepared
- * reference voice: TextEncoder (nn/text.py:16-44) -> txt_seq, txt_pool; base = txt_pool + frame sinusoid;
+ * reference voice (sopro_prefill_run) or each bring their own (sopro_prefill_run_voices): TextEncoder (nn/text.py:16-44) -> txt_seq, txt_pool; base = txt_pool + frame sinusoid;
  * SpeakerFiLM (nn/speaker.py:64-85); RefXAttnStack with cached K/V (nn/ref.py:57-108, 111-160); cond_norm -> cond_ar.
  * fp32 (cond_ar / txt_seq feed the id-exact AR kernel).  HOST fp32 weight pointers, state_dict layouts.
  * prepare_reference (once per voice: Token2SV, reference encoder, K/V projections) is sopro_refprep_* below.
@@ -476,6 +476,18 @@ int sopro_prefill_destroy(sopro_prefill_t* p);
 int sopro_prefill_run(sopro_prefill_t* p, const int32_t* text_ids, const int32_t* text_len, int B, int Lmax, const float* sv,
                       int sv_shared, const float* const* ref_k, const float* const* ref_v, int Tr, float style_strength,
                       int n_frames, float* txt_seq, float* txt_pool, float* cond_ar, void* stream);
+/* The same prefill for B texts that each bring their own prepared voice (n_voices distinct voices in the call).
+ * DEVICE: text_ids [B, Lmax] i32, text_len [B] i32, sv [n_voices, sv_dim] (row v: voice v's speaker vector); outputs
+ * as sopro_prefill_run.  HOST (reusable as soon as the call returns; the tables are staged into the engine's workspace
+ * on `stream`): voice [B] i32, text b's voice in [0, n_voices); ref_len [n_voices] i32, Tr of each voice in [1, 4096];
+ * ref_k / ref_v [ref_layers * n_voices] device pointers, entry l * n_voices + v = voice v's cached K / V of layer l,
+ * [H, Tr_v, D/H] (PreparedReference.ref_kv_caches[l]).  Utterance b's txt_seq / txt_pool / cond_ar rows are bit-equal
+ * to what sopro_prefill_run computes for the same texts with voice[b]'s reference shared by all of them (sv_shared = 1).
+ * A null pointer, n_voices < 1, a voice index or a Tr out of range return SOPRO_ERR_INVALID before any launch. */
+int sopro_prefill_run_voices(sopro_prefill_t* p, const int32_t* text_ids, const int32_t* text_len, int B, int Lmax,
+                             const int32_t* voice, int n_voices, const float* sv, const int32_t* ref_len,
+                             const float* const* ref_k, const float* const* ref_v, float style_strength, int n_frames,
+                             float* txt_seq, float* txt_pool, float* cond_ar, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Reference preparation: SoproTTSModel.prepare_reference (reference model.py:152-170), once per voice, from the

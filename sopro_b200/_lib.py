@@ -200,6 +200,7 @@ SYMBOLS = {
     "sopro_refprep_run": (_I, [_VP, _VP, _I, _VP, _VP, _VP, _VP, _VP]),
     "sopro_refprep_check": (_I, [_VP, _VP]),
     "sopro_prefill_run": (_I, [_VP, _VP, _VP, _I, _I, _VP, _I, _VP, _VP, _I, C.c_float, _I, _VP, _VP, _VP, _VP]),
+    "sopro_prefill_run_voices": (_I, [_VP, _VP, _VP, _I, _I, _VP, _I, _VP, _VP, _VP, _VP, C.c_float, _I, _VP, _VP, _VP, _VP]),
     "sopro_debug_tc_gemm": (_I, [_VP, _I, C.c_int64, _I, _I, _I, _I, _VP, _I, _VP, _I, _I, _VP, _VP, _VP, _VP, _I, _VP]),
 }
 

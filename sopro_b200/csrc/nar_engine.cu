@@ -809,9 +809,11 @@ __global__ void __launch_bounds__(128) mean_pool_kernel(const float* __restrict_
 
 // one warp per (b, t) row: base = pool[b] + frame_pos[t]; LayerNorm (eps 1e-5, biased variance) * w + bias;
 // y = ln * (1 + s*tanh(gamma[b])) + s*tanh(beta[b])         (film rows [Bf][2D], Bf = B or 1)
+// film_index (per-utterance voices): utterance b reads film row film_index[b] instead
 __global__ void __launch_bounds__(256) film_rows_kernel(const float* __restrict__ pool, const float* __restrict__ fpos,
                                                         const float* __restrict__ ln_w, const float* __restrict__ ln_b,
-                                                        const float* __restrict__ film, int film_shared, float strength,
+                                                        const float* __restrict__ film, int film_shared,
+                                                        const int* __restrict__ film_index, float strength,
                                                         float* __restrict__ y, long long rows, int T, int D) {
   const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
@@ -837,7 +839,7 @@ __global__ void __launch_bounds__(256) film_rows_kernel(const float* __restrict_
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) var += __shfl_xor_sync(0xffffffffu, var, o);
   const float inv = 1.0f / sqrtf(var / (float)D + 1e-5f);
-  const float* f = film + (film_shared ? 0 : b * 2 * D);
+  const float* f = film + (film_index ? (long long)film_index[b] * 2 * D : film_shared ? 0 : b * 2 * D);
   n = 0;
   for (int k = lane; k < D; k += 32, ++n) {
     const float ln = (v[n] - mean) * inv * __ldg(ln_w + k) + __ldg(ln_b + k);
@@ -845,19 +847,18 @@ __global__ void __launch_bounds__(256) film_rows_kernel(const float* __restrict_
   }
 }
 
-// Cached reference cross-attention core + RMS matching, one warp per query row (nn/ref.py:84-101):
+// Cached reference cross-attention core + RMS matching of ONE query row, by one warp (nn/ref.py:84-101):
 //   per head: s_j = q.K_j / sqrt(dh); p = softmax(s); a = sum_j p_j V_j; nan_to_num
 //   a *= clamp(rms(x) / rms(a), 0, 10) over the full row (both heads)
-// K, V: [H][Tr][dh] (one shared reference voice).  Shared memory per warp: q [D] | p [Tr] | a [D].
-__global__ void __launch_bounds__(256) ref_attn_kernel(const float* __restrict__ q, const float* __restrict__ x,
-                                                       const float* __restrict__ Kc, const float* __restrict__ Vc,
-                                                       float* __restrict__ out, long long rows, int D, int H, int Tr) {
-  extern __shared__ float rsm[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long row = (long long)blockIdx.x * 8 + warp;
-  if (row >= rows) return;
+// K, V: [H][Tr][dh] (the row's reference voice).  Shared memory per warp: q [D] | p [Tr] | a [D], in regions sized for
+// Tr_region >= Tr rows of p.  Both attention kernels below run this one instruction sequence, so a row's result depends
+// only on its own voice.
+__device__ __forceinline__ void ref_attn_row(const float* __restrict__ q, const float* __restrict__ x,
+                                             const float* __restrict__ Kc, const float* __restrict__ Vc,
+                                             float* __restrict__ out, long long row, int D, int H, int Tr, int Tr_region,
+                                             float* rsm, int warp, int lane) {
   const int dh = D / H, Trp = (Tr + 3) & ~3;  // padded: the per-warp regions stay 16-byte aligned
-  float* qs = rsm + (size_t)warp * (2 * D + Trp);
+  float* qs = rsm + (size_t)warp * (2 * D + ((Tr_region + 3) & ~3));
   float* ps = qs + D;
   float* as = ps + Trp;
   for (int k = lane; k < D; k += 32) qs[k] = q[row * D + k];
@@ -916,6 +917,31 @@ __global__ void __launch_bounds__(256) ref_attn_kernel(const float* __restrict__
   for (int k = lane; k < D; k += 32) out[row * D + k] = as[k] * sc;
 }
 
+// one shared reference voice: K, V [H][Tr][dh]
+__global__ void __launch_bounds__(256) ref_attn_kernel(const float* __restrict__ q, const float* __restrict__ x,
+                                                       const float* __restrict__ Kc, const float* __restrict__ Vc,
+                                                       float* __restrict__ out, long long rows, int D, int H, int Tr) {
+  extern __shared__ float rsm[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = (long long)blockIdx.x * 8 + warp;
+  if (row >= rows) return;
+  ref_attn_row(q, x, Kc, Vc, out, row, D, H, Tr, Tr, rsm, warp, lane);
+}
+
+// a voice per utterance: row r belongs to utterance b = r / T and reads voice v = voice[b]: K, V = Kv[v], Vv[v]
+// ([H][tr[v]][dh], this layer's).  The per-warp shared-memory regions are sized by Trmax, the largest tr[v].
+__global__ void __launch_bounds__(256) ref_attn_voices_kernel(const float* __restrict__ q, const float* __restrict__ x,
+                                                              const float* const* __restrict__ Kv, const float* const* __restrict__ Vv,
+                                                              const int* __restrict__ voice, const int* __restrict__ tr,
+                                                              float* __restrict__ out, long long rows, int T, int D, int H, int Trmax) {
+  extern __shared__ float rsm[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = (long long)blockIdx.x * 8 + warp;
+  if (row >= rows) return;
+  const int v = voice[(int)row / T];  // rows < 2^30 (sopro_prefill_run_voices checks B * n_frames)
+  ref_attn_row(q, x, Kv[v], Vv[v], out, row, D, H, tr[v], Trmax, rsm, warp, lane);
+}
+
 }  // namespace pstage
 
 struct sopro_prefill {
@@ -932,7 +958,152 @@ struct sopro_prefill {
   } ref[SOPRO_PREFILL_MAX_REF_LAYERS]{};
   float* ws = nullptr;
   size_t ws_bytes = 0;
+  // pinned staging of sopro_prefill_run_voices' voice tables: the upload is asynchronous, pin_done marks when it has
+  // read the buffer
+  char* pin = nullptr;
+  size_t pin_bytes = 0;
+  cudaEvent_t pin_done = nullptr;
 };
+
+namespace pstage {
+
+// The voices of sopro_prefill_run_voices, as the caller passed them (host arrays).
+struct Voices {
+  int n;                  // voices
+  const int32_t* voice;   // [B] voice of each text
+  const int32_t* tr;      // [n] Tr of each voice
+  const float* const* k;  // [ref_layers * n] device pointers, entry l * n + v
+  const float* const* v;
+};
+
+// Both prefill entry points after validation.  mv == nullptr: sopro_prefill_run (sv [B or 1], ref_k / ref_v / Tr of
+// the shared voice).  Otherwise a voice per text: sv [mv->n][sv_dim], K / V and Tr from mv; the voice tables are staged
+// in the workspace, and each voice's FiLM row is computed by the skinny kernel like a shared voice's (see below).
+int prefill_run(sopro_prefill* p, const int32_t* text_ids, const int32_t* text_len, int B, int Lmax, const float* sv, int sv_shared,
+                const float* const* ref_k, const float* const* ref_v, int Tr, const Voices* mv, float style_strength, int n_frames,
+                float* txt_seq, float* txt_pool, float* cond_ar, void* stream) {
+  const sopro_prefill_config_t& c = p->cfg;
+  const int D = c.d_model, SV = c.sv_dim, H = c.ref_heads;
+  PCK(cudaSetDevice(p->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const long long Mt = (long long)B * Lmax, Mc = (long long)B * n_frames;
+  auto al = [](size_t x) { return (x + 63) / 64 * 64; };
+  const size_t rows = (size_t)std::max(Mt, Mc);
+  const int Bf = mv ? mv->n : sv_shared ? 1 : B;  // FiLM rows
+  const int Bw = mv ? mv->n : B;
+  // voice tables (mv): K / V pointers [ref_layers][2][n] | voice [B] | tr [n]
+  const size_t n_ptr = mv ? (size_t)c.ref_layers * 2 * mv->n : 0, tab_bytes = mv ? n_ptr * 8 + ((size_t)B + mv->n) * 4 : 0;
+  const size_t need = (al(rows * D) * 3 + al(rows * 4 * D) + al((size_t)Bw * D) + al((size_t)Bw * 2 * D) + al((tab_bytes + 3) / 4)) * 4;
+  if (p->ws_bytes < need) {
+    PCK(cudaStreamSynchronize(st));
+    cudaFree(p->ws);
+    p->ws = nullptr;
+    p->ws_bytes = 0;
+    cudaError_t e = cudaMalloc(&p->ws, need);
+    if (e != cudaSuccess) return fail(SOPRO_ERR_CUDA, "prefill workspace %zu MB: %s", need >> 20, cudaGetErrorString(e));
+    p->ws_bytes = need;
+  }
+  float* x = p->ws;
+  float* h = x + al(rows * D);
+  float* q = h + al(rows * D);
+  float* hid = q + al(rows * D);
+  float* fmid = hid + al(rows * 4 * D);      // [Bf][D] FiLM hidden
+  float* film = fmid + al((size_t)Bw * D);   // [Bf][2D]
+  float* tab = film + al((size_t)Bw * 2 * D);
+  const float* const* tab_kv = reinterpret_cast<const float* const*>(tab);
+  const int* tab_voice = reinterpret_cast<const int*>(reinterpret_cast<const char*>(tab) + n_ptr * 8);
+  const int* tab_tr = mv ? tab_voice + B : nullptr;
+  int Tra = Tr;  // the largest Tr of the call
+  if (mv) {
+    if (!p->pin_done) PCK(cudaEventCreateWithFlags(&p->pin_done, cudaEventDisableTiming));
+    else PCK(cudaEventSynchronize(p->pin_done));  // the previous call's upload has read the staging buffer (normally long ago)
+    if (p->pin_bytes < tab_bytes) {
+      cudaFreeHost(p->pin);
+      p->pin = nullptr;
+      p->pin_bytes = 0;
+      PCK(cudaMallocHost(reinterpret_cast<void**>(&p->pin), tab_bytes));
+      p->pin_bytes = tab_bytes;
+    }
+    const float** kv = reinterpret_cast<const float**>(p->pin);
+    for (int l = 0; l < c.ref_layers; ++l)
+      for (int v = 0; v < mv->n; ++v) {
+        kv[(size_t)(2 * l) * mv->n + v] = mv->k[(size_t)l * mv->n + v];
+        kv[(size_t)(2 * l + 1) * mv->n + v] = mv->v[(size_t)l * mv->n + v];
+      }
+    memcpy(p->pin + n_ptr * 8, mv->voice, (size_t)B * 4);
+    memcpy(p->pin + n_ptr * 8 + (size_t)B * 4, mv->tr, (size_t)mv->n * 4);
+    PCK(cudaMemcpyAsync(tab, p->pin, tab_bytes, cudaMemcpyHostToDevice, st));
+    PCK(cudaEventRecord(p->pin_done, st));
+    Tra = *std::max_element(mv->tr, mv->tr + mv->n);
+  }
+  const float* W = p->dev;
+  int rc;
+  // ---- text encoder
+  text_embed_kernel<<<dim3(Lmax, B), 128, 0, st>>>(text_ids, text_len, W + p->text_emb, W + p->text_pos, x, Lmax, D, c.text_vocab);
+  PCK(cudaGetLastError());
+  for (int i = 0; i < c.n_layers_text; ++i)
+    if ((rc = ssm_block(W, p->blk[i], x, h, hid, text_len, B, Lmax, D, c.text_kernel, 1, false, st))) return rc;
+  dense::rmsnorm_rows_kernel<<<(unsigned)((Mt + 7) / 8), 256, 0, st>>>(x, W + p->text_norm_w, nullptr, nullptr, txt_seq, Mt, D);
+  PCK(cudaGetLastError());
+  mean_pool_kernel<<<B, 128, 0, st>>>(txt_seq, text_len, txt_pool, Lmax, D);
+  PCK(cudaGetLastError());
+  // ---- FiLM parameters from the speaker vector(s).  Per voice in launches of at most 16 rows: the skinny kernel stages
+  // 16 rows whatever M is and reduces every row through the same butterfly, so a voice's row is bit-equal to the M = 1
+  // launch of a shared voice.  One launch of more than 16 rows would take the tile kernel, which sums in another order.
+  const int chunk = mv ? dense::kSkinnyRows : Bf;
+  for (int r0 = 0; r0 < Bf; r0 += chunk) {
+    const int m = std::min(chunk, Bf - r0);
+    dense::DenseOp g{};
+    g.A = sv + (size_t)r0 * SV; g.W = W + p->film_w0; g.bias = W + p->film_b0; g.C = fmid + (size_t)r0 * D; g.M = m; g.N = D; g.K = SV;
+    g.ldc = D; g.epi = dense::EPI_GELU;
+    if ((rc = launch_dense(g, 1, st))) return rc;
+    g = dense::DenseOp{};
+    g.A = fmid + (size_t)r0 * D; g.W = W + p->film_w2; g.bias = W + p->film_b2; g.C = film + (size_t)r0 * 2 * D; g.M = m; g.N = 2 * D;
+    g.K = D; g.ldc = 2 * D; g.epi = dense::EPI_BIAS;
+    if ((rc = launch_dense(g, 1, st))) return rc;
+  }
+  film_rows_kernel<<<(unsigned)((Mc + 7) / 8), 256, 0, st>>>(txt_pool, W + p->frame_pos, W + p->film_ln_w, W + p->film_ln_b, film, sv_shared ? 1 : 0,
+                                                            mv ? tab_voice : nullptr, style_strength, x, Mc, n_frames, D);
+  PCK(cudaGetLastError());
+  // ---- reference cross-attention stack
+  const size_t rsmem = (size_t)8 * (2 * D + ((Tra + 3) & ~3)) * 4;
+  if (c.ref_layers > 0 && rsmem > 48 * 1024) {
+    static bool attr = false, attr_voices = false;
+    bool& done = mv ? attr_voices : attr;
+    if (!done) {
+      if (mv) PCK(cudaFuncSetAttribute(ref_attn_voices_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      else PCK(cudaFuncSetAttribute(ref_attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      done = true;
+    }
+  }
+  for (int i = 0; i < c.ref_layers; ++i) {
+    dense::DenseOp g{};
+    g.A = x; g.W = W + p->ref[i].q_w; g.norm_w = W + p->ref[i].nq_w; g.C = q; g.M = (int)Mc; g.N = D; g.K = D; g.ldc = D; g.epi = dense::EPI_BIAS;
+    if ((rc = launch_dense(g, 1, st))) return rc;
+    if (mv)
+      ref_attn_voices_kernel<<<(unsigned)((Mc + 7) / 8), 256, rsmem, st>>>(q, x, tab_kv + (size_t)(2 * i) * mv->n, tab_kv + (size_t)(2 * i + 1) * mv->n,
+                                                                           tab_voice, tab_tr, h, Mc, n_frames, D, H, Tra);
+    else
+      ref_attn_kernel<<<(unsigned)((Mc + 7) / 8), 256, rsmem, st>>>(q, x, ref_k[i], ref_v[i], h, Mc, D, H, Tr);
+    PCK(cudaGetLastError());
+    g = dense::DenseOp{};
+    g.A = h; g.W = W + p->ref[i].o_w; g.R = x; g.C = x; g.M = (int)Mc; g.N = D; g.K = D; g.ldc = D; g.epi = dense::EPI_RES_GATE;
+    g.gate = p->ref[i].gate_eff;
+    if ((rc = launch_dense(g, 1, st))) return rc;
+  }
+  dense::rmsnorm_rows_kernel<<<(unsigned)((Mc + 7) / 8), 256, 0, st>>>(x, W + p->cond_norm_w, nullptr, nullptr, cond_ar, Mc, D);
+  PCK(cudaGetLastError());
+  return SOPRO_OK;
+}
+
+int check_batch(const sopro_prefill* p, int B, int Lmax, int n_frames) {
+  const sopro_prefill_config_t& c = p->cfg;
+  if (B < 1 || Lmax < 1 || Lmax > c.max_text_len || n_frames < 1 || n_frames > c.max_frames_pos || (long long)B * n_frames > 0x3fffffffLL)
+    return fail(SOPRO_ERR_INVALID, "bad B=%d Lmax=%d (max %d) n_frames=%d (max %d)", B, Lmax, c.max_text_len, n_frames, c.max_frames_pos);
+  return SOPRO_OK;
+}
+
+}  // namespace pstage
 
 extern "C" {
 
@@ -995,6 +1166,11 @@ int sopro_prefill_create(const sopro_prefill_config_t* cfg, const sopro_prefill_
 int sopro_prefill_destroy(sopro_prefill_t* p) {
   if (!p) return SOPRO_OK;
   cudaSetDevice(p->device);
+  if (p->pin_done) {
+    cudaEventSynchronize(p->pin_done);
+    cudaEventDestroy(p->pin_done);
+  }
+  cudaFreeHost(p->pin);
   cudaFree(p->dev);
   cudaFree(p->ws);
   delete p;
@@ -1005,77 +1181,33 @@ int sopro_prefill_run(sopro_prefill_t* p, const int32_t* text_ids, const int32_t
                       int sv_shared, const float* const* ref_k, const float* const* ref_v, int Tr, float style_strength, int n_frames,
                       float* txt_seq, float* txt_pool, float* cond_ar, void* stream) {
   if (!p || !text_ids || !text_len || !sv || !txt_seq || !txt_pool || !cond_ar) return fail(SOPRO_ERR_INVALID, "null argument");
-  const sopro_prefill_config_t& c = p->cfg;
-  const int D = c.d_model, SV = c.sv_dim, H = c.ref_heads;
-  if (B < 1 || Lmax < 1 || Lmax > c.max_text_len || n_frames < 1 || n_frames > c.max_frames_pos || (long long)B * n_frames > 0x3fffffffLL)
-    return fail(SOPRO_ERR_INVALID, "bad B=%d Lmax=%d (max %d) n_frames=%d (max %d)", B, Lmax, c.max_text_len, n_frames, c.max_frames_pos);
-  if (c.ref_layers > 0 && (!ref_k || !ref_v || Tr < 1 || Tr > 4096)) return fail(SOPRO_ERR_INVALID, "reference K/V missing or Tr=%d out of range", Tr);
-  PCK(cudaSetDevice(p->device));
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const long long Mt = (long long)B * Lmax, Mc = (long long)B * n_frames;
-  auto al = [](size_t x) { return (x + 63) / 64 * 64; };
-  const size_t rows = (size_t)std::max(Mt, Mc);
-  const size_t need = (al(rows * D) * 3 + al(rows * 4 * D) + al((size_t)B * D) + al((size_t)B * 2 * D)) * 4;
-  if (p->ws_bytes < need) {
-    PCK(cudaStreamSynchronize(st));
-    cudaFree(p->ws);
-    p->ws = nullptr;
-    p->ws_bytes = 0;
-    cudaError_t e = cudaMalloc(&p->ws, need);
-    if (e != cudaSuccess) return fail(SOPRO_ERR_CUDA, "prefill workspace %zu MB: %s", need >> 20, cudaGetErrorString(e));
-    p->ws_bytes = need;
-  }
-  float* x = p->ws;
-  float* h = x + al(rows * D);
-  float* q = h + al(rows * D);
-  float* hid = q + al(rows * D);
-  float* fmid = hid + al(rows * 4 * D);  // [B][D] FiLM hidden
-  float* film = fmid + al((size_t)B * D);  // [B][2D]
-  const float* W = p->dev;
   int rc;
-  // ---- text encoder
-  text_embed_kernel<<<dim3(Lmax, B), 128, 0, st>>>(text_ids, text_len, W + p->text_emb, W + p->text_pos, x, Lmax, D, c.text_vocab);
-  PCK(cudaGetLastError());
-  for (int i = 0; i < c.n_layers_text; ++i)
-    if ((rc = ssm_block(W, p->blk[i], x, h, hid, text_len, B, Lmax, D, c.text_kernel, 1, false, st))) return rc;
-  dense::rmsnorm_rows_kernel<<<(unsigned)((Mt + 7) / 8), 256, 0, st>>>(x, W + p->text_norm_w, nullptr, nullptr, txt_seq, Mt, D);
-  PCK(cudaGetLastError());
-  mean_pool_kernel<<<B, 128, 0, st>>>(txt_seq, text_len, txt_pool, Lmax, D);
-  PCK(cudaGetLastError());
-  // ---- FiLM parameters from the speaker vector(s)
-  const int Bf = sv_shared ? 1 : B;
-  dense::DenseOp g{};
-  g.A = sv; g.W = W + p->film_w0; g.bias = W + p->film_b0; g.C = fmid; g.M = Bf; g.N = D; g.K = SV; g.ldc = D; g.epi = dense::EPI_GELU;
-  if ((rc = launch_dense(g, 1, st))) return rc;
-  g = dense::DenseOp{};
-  g.A = fmid; g.W = W + p->film_w2; g.bias = W + p->film_b2; g.C = film; g.M = Bf; g.N = 2 * D; g.K = D; g.ldc = 2 * D; g.epi = dense::EPI_BIAS;
-  if ((rc = launch_dense(g, 1, st))) return rc;
-  film_rows_kernel<<<(unsigned)((Mc + 7) / 8), 256, 0, st>>>(txt_pool, W + p->frame_pos, W + p->film_ln_w, W + p->film_ln_b, film, sv_shared ? 1 : 0,
-                                                            style_strength, x, Mc, n_frames, D);
-  PCK(cudaGetLastError());
-  // ---- reference cross-attention stack
-  const size_t rsmem = (size_t)8 * (2 * D + ((Tr + 3) & ~3)) * 4;
-  if (c.ref_layers > 0 && rsmem > 48 * 1024) {
-    static bool attr = false;
-    if (!attr) {
-      PCK(cudaFuncSetAttribute(ref_attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      attr = true;
-    }
-  }
-  for (int i = 0; i < c.ref_layers; ++i) {
-    g = dense::DenseOp{};
-    g.A = x; g.W = W + p->ref[i].q_w; g.norm_w = W + p->ref[i].nq_w; g.C = q; g.M = (int)Mc; g.N = D; g.K = D; g.ldc = D; g.epi = dense::EPI_BIAS;
-    if ((rc = launch_dense(g, 1, st))) return rc;
-    ref_attn_kernel<<<(unsigned)((Mc + 7) / 8), 256, rsmem, st>>>(q, x, ref_k[i], ref_v[i], h, Mc, D, H, Tr);
-    PCK(cudaGetLastError());
-    g = dense::DenseOp{};
-    g.A = h; g.W = W + p->ref[i].o_w; g.R = x; g.C = x; g.M = (int)Mc; g.N = D; g.K = D; g.ldc = D; g.epi = dense::EPI_RES_GATE;
-    g.gate = p->ref[i].gate_eff;
-    if ((rc = launch_dense(g, 1, st))) return rc;
-  }
-  dense::rmsnorm_rows_kernel<<<(unsigned)((Mc + 7) / 8), 256, 0, st>>>(x, W + p->cond_norm_w, nullptr, nullptr, cond_ar, Mc, D);
-  PCK(cudaGetLastError());
-  return SOPRO_OK;
+  if ((rc = check_batch(p, B, Lmax, n_frames))) return rc;
+  if (p->cfg.ref_layers > 0 && (!ref_k || !ref_v || Tr < 1 || Tr > 4096)) return fail(SOPRO_ERR_INVALID, "reference K/V missing or Tr=%d out of range", Tr);
+  return prefill_run(p, text_ids, text_len, B, Lmax, sv, sv_shared, ref_k, ref_v, Tr, nullptr, style_strength, n_frames, txt_seq, txt_pool,
+                     cond_ar, stream);
+}
+
+int sopro_prefill_run_voices(sopro_prefill_t* p, const int32_t* text_ids, const int32_t* text_len, int B, int Lmax, const int32_t* voice,
+                             int n_voices, const float* sv, const int32_t* ref_len, const float* const* ref_k, const float* const* ref_v,
+                             float style_strength, int n_frames, float* txt_seq, float* txt_pool, float* cond_ar, void* stream) {
+  if (!p || !text_ids || !text_len || !voice || !sv || !ref_len || !txt_seq || !txt_pool || !cond_ar)
+    return fail(SOPRO_ERR_INVALID, "null argument");
+  int rc;
+  if ((rc = check_batch(p, B, Lmax, n_frames))) return rc;
+  if (n_voices < 1) return fail(SOPRO_ERR_INVALID, "n_voices=%d: at least one voice is needed", n_voices);
+  for (int b = 0; b < B; ++b)
+    if (voice[b] < 0 || voice[b] >= n_voices) return fail(SOPRO_ERR_INVALID, "voice[%d]=%d out of range [0, %d)", b, voice[b], n_voices);
+  for (int v = 0; v < n_voices; ++v)
+    if (ref_len[v] < 1 || ref_len[v] > 4096) return fail(SOPRO_ERR_INVALID, "ref_len[%d]=%d out of range [1, 4096]", v, ref_len[v]);
+  const int RL = p->cfg.ref_layers;
+  if (RL > 0 && (!ref_k || !ref_v)) return fail(SOPRO_ERR_INVALID, "reference K/V tables missing");
+  for (long long i = 0; i < (long long)RL * n_voices; ++i)
+    if (!ref_k[i] || !ref_v[i])
+      return fail(SOPRO_ERR_INVALID, "reference K/V of layer %lld, voice %lld is null", i / n_voices, i % n_voices);
+  const Voices mv{n_voices, voice, ref_len, ref_k, ref_v};
+  return prefill_run(p, text_ids, text_len, B, Lmax, sv, 0, nullptr, nullptr, 0, &mv, style_strength, n_frames, txt_seq, txt_pool, cond_ar,
+                     stream);
 }
 
 }  // extern "C"

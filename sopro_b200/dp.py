@@ -76,10 +76,15 @@ class DataParallelTTS:
     def shard(self, n_items: int) -> Tuple[int, int]:
         return shard_range(n_items, self.rank, self.world)
 
-    def synthesize_batch(self, texts: Sequence[str], *, ref, seeds: Optional[Sequence[int]] = None, **kw):
-        """-> (waveforms of THIS rank's utterances, (lo, hi)): texts[lo:hi] of the global batch."""
+    def synthesize_batch(self, texts: Sequence[str], *, ref=None, refs=None, seeds: Optional[Sequence[int]] = None, **kw):
+        """-> (waveforms of THIS rank's utterances, (lo, hi)): texts[lo:hi] of the global batch, with their seeds and,
+        for a voice per text, their refs[lo:hi]."""
+        if refs is not None and len(refs) != len(texts):
+            raise ValueError(f"refs has {len(refs)} entries for {len(texts)} texts")
         lo, hi = self.shard(len(texts))
         if hi <= lo:
             return [], (lo, hi)
+        if refs is not None:
+            kw["refs"] = list(refs[lo:hi])
         wavs = self.tts.synthesize_batch(list(texts[lo:hi]), ref=ref, seeds=None if seeds is None else list(seeds[lo:hi]), **kw)
         return wavs, (lo, hi)

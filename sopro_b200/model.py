@@ -267,19 +267,36 @@ class SoproModel:
         return self.prepare_conditioning_batch([text_ids_1d], ref, max_frames=max_frames, style_strength=style_strength)[0]
 
     @torch.no_grad()
-    def prepare_conditioning_batch(self, text_ids: Sequence[torch.Tensor], ref: PreparedReference, *, max_frames: int,
+    def prepare_conditioning_batch(self, text_ids: Sequence[torch.Tensor], ref: Optional[PreparedReference] = None, *,
+                                   refs: Optional[Sequence[PreparedReference]] = None, max_frames: int,
                                    style_strength: float = 1.2) -> List[Dict[str, torch.Tensor]]:
-        """NEW (the reference is batch-1): the prefill of B texts that share one prepared reference in ONE pass; element i
-        is the `prep` dict of model.py:210-216 for text i (views into the batch tensors)."""
-        txt_seq, lens, txt_pool, cond = self.prefill.run(text_ids, ref, n_frames=int(max_frames) + 1, style_strength=float(style_strength))
-        sv = ref.sv_ref.to(self.device)
-        if sv.dim() == 1:
-            sv = sv.unsqueeze(0)
+        """NEW (the reference is batch-1): the prefill of B texts in ONE pass, all with the prepared reference `ref`, or
+        text i with its own `refs[i]` (exactly one of the two); element i is the `prep` dict of model.py:210-216 for
+        text i (views into the batch tensors)."""
+        txt_seq, lens, txt_pool, cond = self.prefill_batch(text_ids, ref, refs, n_frames=int(max_frames) + 1,
+                                                           style_strength=float(style_strength))
+        svs: Dict[int, torch.Tensor] = {}
         out = []
         for i, L in enumerate(lens):
+            r = ref if refs is None else refs[i]
+            if id(r) not in svs:
+                sv = r.sv_ref.to(self.device)
+                svs[id(r)] = sv.unsqueeze(0) if sv.dim() == 1 else sv
             out.append({"txt_seq": txt_seq[i: i + 1, :L], "text_mask": torch.ones((1, L), dtype=torch.bool, device=self.device),
-                        "txt_pool": txt_pool[i: i + 1], "sv_ref": sv, "cond_ar": cond[i: i + 1]})
+                        "txt_pool": txt_pool[i: i + 1], "sv_ref": svs[id(r)], "cond_ar": cond[i: i + 1]})
         return out
+
+    def prefill_batch(self, text_ids: Sequence[torch.Tensor], ref: Optional[PreparedReference],
+                      refs: Optional[Sequence[PreparedReference]], *, n_frames: int, style_strength: float):
+        """The batched CUDA prefill with one voice for every text (`ref`) or a voice per text (`refs`, told apart by
+        object identity); exactly one of the two.  -> txt_seq [B, Lmax, D], lens, txt_pool [B, D], cond_ar [B, n_frames, D]."""
+        if (ref is None) == (refs is None):
+            raise ValueError("pass exactly one of ref= (one voice for every text) or refs= (one voice per text)")
+        if refs is None:
+            return self.prefill.run(text_ids, ref, n_frames=n_frames, style_strength=style_strength)
+        if len(refs) != len(text_ids):
+            raise ValueError(f"refs has {len(refs)} entries for {len(text_ids)} texts")
+        return self.prefill.run_voices(text_ids, list(refs), n_frames=n_frames, style_strength=style_strength)
 
     @torch.no_grad()
     def nar_refine(self, cond_seq: torch.Tensor, rvq1_1xT: torch.Tensor, lens: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -590,15 +607,18 @@ class SoproTTS:
         return self.codec.decode_full(tokens_tq)
 
     @torch.inference_mode()
-    def synthesize_batch(self, texts: Sequence[str], *, ref: PreparedReference, max_frames: int = 400, top_p: float = 0.9,
+    def synthesize_batch(self, texts: Sequence[str], *, ref: Optional[PreparedReference] = None,
+                         refs: Optional[Sequence[PreparedReference]] = None, max_frames: int = 400, top_p: float = 0.9,
                          temperature: float = 1.05, anti_loop: bool = True, style_strength: Optional[float] = None,
                          min_gen_frames: Optional[int] = None, seeds: Optional[Sequence[int]] = None) -> List[torch.Tensor]:
-        """NEW: B texts with one shared prepared reference -> B waveforms [1, 1, N_i].  One batched prefill, one
-        persistent AR launch, one ragged NAR pass, padded Mimi decodes; utterance i equals synthesize(texts[i], seed=seeds[i])."""
+        """NEW: B texts -> B waveforms [1, 1, N_i], all in the voice of one prepared reference `ref`, or text i in the
+        voice of its own `refs[i]` (exactly one of the two; a server caching one PreparedReference per user passes the
+        cached objects, repeated ones are recognised by identity).  One batched prefill, one persistent AR launch, one
+        ragged NAR pass, padded Mimi decodes; utterance i equals synthesize(texts[i], ref=(ref or refs[i]), seed=seeds[i])."""
         st = float(style_strength if style_strength is not None else self.cfg.style_strength)
         model = self.model
         ids = [self.encode_text(t) for t in texts]
-        txt_seq, lens, _pool, cond = model.prefill.run(ids, ref, n_frames=int(max_frames) + 1, style_strength=st)
+        txt_seq, lens, _pool, cond = model.prefill_batch(ids, ref, refs, n_frames=int(max_frames) + 1, style_strength=st)
         toks, n = model.ar_generate_tensors(cond, txt_seq, lens, max_frames=max_frames, top_p=top_p, temperature=temperature,
                                             anti_loop=anti_loop, min_gen_frames=min_gen_frames, seeds=seeds)
         eos, B = model.eos_id, len(texts)

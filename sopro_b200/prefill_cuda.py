@@ -1,6 +1,7 @@
 """Host side of the CUDA prefill (libsopro_b200.so: sopro_prefill_*; reference model.py:172-216): text encoder,
-FiLM, cached reference cross-attention and cond_norm for B texts sharing one prepared reference voice -- and of the
-once-per-voice reference preparation in front of it (sopro_refprep_*; reference model.py:152-170)."""
+FiLM, cached reference cross-attention and cond_norm for B texts that share one prepared reference voice (`run`) or
+each bring their own (`run_voices`) -- and of the once-per-voice reference preparation in front of it (sopro_refprep_*;
+reference model.py:152-170)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -54,12 +55,65 @@ class PrefillEngine:
         _lib.check(self.lib.sopro_prefill_create(C.byref(c), C.byref(w), self.device.index, C.byref(h)))
         self._h = h
         self.D, self.n_ref = int(cfg.d_model), int(c.ref_layers)
-        self.max_text_len = int(c.max_text_len)
+        self.max_text_len, self.sv_dim = int(c.max_text_len), int(c.sv_dim)
         del keep
 
     def run(self, text_ids: Sequence[torch.Tensor], ref, *, n_frames: int, style_strength: float):
         """text_ids: B 1-D id tensors; ref: PreparedReference (shared).  -> txt_seq [B, Lmax, D], lens (list),
         txt_pool [B, D], cond_ar [B, n_frames, D] on the device."""
+        B = len(text_ids)
+        ids, ln, lens, Lmax = self._texts(text_ids)
+        sv = ref.sv_ref.to(self.device, torch.float32).reshape(-1, ref.sv_ref.shape[-1]).contiguous()
+        ks, vs, Tr = self._ref_kv(ref)
+        kp = (C.c_void_p * max(1, self.n_ref))(*[int(k.data_ptr()) for k in ks])
+        vp = (C.c_void_p * max(1, self.n_ref))(*[int(v.data_ptr()) for v in vs])
+        txt_seq = torch.empty((B, Lmax, self.D), dtype=torch.float32, device=self.device)
+        txt_pool = torch.empty((B, self.D), dtype=torch.float32, device=self.device)
+        cond = torch.empty((B, int(n_frames), self.D), dtype=torch.float32, device=self.device)
+        _lib.check(self.lib.sopro_prefill_run(self._h, ids.data_ptr(), ln.data_ptr(), B, Lmax, sv.data_ptr(), 1 if sv.shape[0] == 1 else 0,
+                                              kp, vp, Tr, float(style_strength), int(n_frames), txt_seq.data_ptr(), txt_pool.data_ptr(),
+                                              cond.data_ptr(), int(torch.cuda.current_stream(self.device).cuda_stream)))
+        self._keep = (ids, ln, sv, ks, vs)  # alive until the stream has consumed them
+        return txt_seq, lens, txt_pool, cond
+
+    def run_voices(self, text_ids: Sequence[torch.Tensor], refs: Sequence, *, n_frames: int, style_strength: float):
+        """text_ids: B 1-D id tensors; refs: B PreparedReference, text i conditioned on refs[i] (the same object may
+        appear several times: voices are told apart by identity).  -> as `run`.  Utterance i is bit-equal to `run` on
+        the same texts with refs[i] shared by all of them."""
+        B = len(text_ids)
+        if len(refs) != B:
+            raise ValueError(f"{len(refs)} references for {B} texts")
+        slot: Dict[int, int] = {}
+        voices: list = []
+        voice = []
+        for r in refs:
+            if id(r) not in slot:
+                slot[id(r)] = len(voices)
+                voices.append(r)
+            voice.append(slot[id(r)])
+        ids, ln, lens, Lmax = self._texts(text_ids)
+        nv = len(voices)
+        sv = torch.stack([r.sv_ref.to(self.device, torch.float32).reshape(-1) for r in voices])
+        if sv.shape[1] != self.sv_dim:
+            raise ValueError(f"a prepared reference holds ONE speaker vector of {self.sv_dim} values")
+        kv = [self._ref_kv(r) for r in voices]  # per voice: ([K of each layer], [V of each layer], Tr)
+        # entry l * n_voices + v: voice v's K / V of layer l (each voice's own tensors, no packing copy)
+        kp = (C.c_void_p * max(1, self.n_ref * nv))(*[int(kv[v][0][l].data_ptr()) for l in range(self.n_ref) for v in range(nv)])
+        vp = (C.c_void_p * max(1, self.n_ref * nv))(*[int(kv[v][1][l].data_ptr()) for l in range(self.n_ref) for v in range(nv)])
+        voice_c = (C.c_int32 * B)(*voice)
+        tr_c = (C.c_int32 * nv)(*[t for _k, _v, t in kv])
+        txt_seq = torch.empty((B, Lmax, self.D), dtype=torch.float32, device=self.device)
+        txt_pool = torch.empty((B, self.D), dtype=torch.float32, device=self.device)
+        cond = torch.empty((B, int(n_frames), self.D), dtype=torch.float32, device=self.device)
+        _lib.check(self.lib.sopro_prefill_run_voices(self._h, ids.data_ptr(), ln.data_ptr(), B, Lmax, voice_c, nv, sv.data_ptr(), tr_c,
+                                                     kp, vp, float(style_strength), int(n_frames), txt_seq.data_ptr(),
+                                                     txt_pool.data_ptr(), cond.data_ptr(),
+                                                     int(torch.cuda.current_stream(self.device).cuda_stream)))
+        self._keep = (ids, ln, sv, kv)  # alive until the stream has consumed them
+        return txt_seq, lens, txt_pool, cond
+
+    def _texts(self, text_ids: Sequence[torch.Tensor]):
+        """B 1-D id tensors -> padded ids [B, Lmax] and lengths [B] on the device, lens, Lmax"""
         B = len(text_ids)
         lens = [int(t.numel()) for t in text_ids]
         if min(lens) < 1:
@@ -72,7 +126,10 @@ class PrefillEngine:
             ids[i, : lens[i]] = t.to("cpu", torch.int32)
         ids = ids.to(self.device, non_blocking=True)
         ln = torch.tensor(lens, dtype=torch.int32).to(self.device, non_blocking=True)
-        sv = ref.sv_ref.to(self.device, torch.float32).reshape(-1, ref.sv_ref.shape[-1]).contiguous()
+        return ids, ln, lens, Lmax
+
+    def _ref_kv(self, ref):
+        """One prepared voice's cached K / V per layer as contiguous fp32 [H, Tr, D/H] device tensors, and Tr."""
         ks: List[torch.Tensor] = []
         vs: List[torch.Tensor] = []
         Tr = 1
@@ -88,16 +145,7 @@ class PrefillEngine:
             ks.append(k.contiguous())
             vs.append(v.contiguous())
             Tr = int(k.shape[1])
-        kp = (C.c_void_p * max(1, self.n_ref))(*[int(k.data_ptr()) for k in ks])
-        vp = (C.c_void_p * max(1, self.n_ref))(*[int(v.data_ptr()) for v in vs])
-        txt_seq = torch.empty((B, Lmax, self.D), dtype=torch.float32, device=self.device)
-        txt_pool = torch.empty((B, self.D), dtype=torch.float32, device=self.device)
-        cond = torch.empty((B, int(n_frames), self.D), dtype=torch.float32, device=self.device)
-        _lib.check(self.lib.sopro_prefill_run(self._h, ids.data_ptr(), ln.data_ptr(), B, Lmax, sv.data_ptr(), 1 if sv.shape[0] == 1 else 0,
-                                              kp, vp, Tr, float(style_strength), int(n_frames), txt_seq.data_ptr(), txt_pool.data_ptr(),
-                                              cond.data_ptr(), int(torch.cuda.current_stream(self.device).cuda_stream)))
-        self._keep = (ids, ln, sv, ks, vs)  # alive until the stream has consumed them
-        return txt_seq, lens, txt_pool, cond
+        return ks, vs, Tr
 
     def close(self) -> None:
         if getattr(self, "_h", None):
